@@ -2,7 +2,7 @@
 """bench.py — headline benchmark of the hot path (BASELINE.json configs[1]):
 threshold -> seeded flood-fill region grow -> marching cubes on a 512^3 int16 CT phantom.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).
 
@@ -117,6 +117,30 @@ def cpu_step(vol, seed, threads, want_arrays=False):
     if want_arrays:
         return count, ntri, mm, out
     return count, ntri
+
+
+DUMP_KEEP = 1 << 20
+
+
+def dump_outputs(dirname, outputs, suffix=""):
+    """--dump-outputs: each output of the last timed step as DIR/<name><suffix>.npy, masks and vertices
+    as float32, triangle indices as float64 (exact). An output with more than DUMP_KEEP voxels (masks)
+    or rows (mesh arrays) keeps DUMP_KEEP of them at fixed, seeded positions, in index order; each mask
+    also gets its exact per-plane sums (<name>_plane_sums), which catch what the sample misses. About
+    44 MiB in all."""
+    import torch
+    d = Path(dirname)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in outputs.items():
+        flat = t.reshape(-1) if t.dim() == 3 else t
+        if flat.shape[0] > DUMP_KEEP:
+            idx = np.sort(np.random.default_rng(0).choice(flat.shape[0], DUMP_KEEP, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        wide = t.dtype in (torch.int32, torch.int64)
+        np.save(d / f"{name}{suffix}.npy", flat.to(torch.float64 if wide else torch.float32).cpu().numpy())
+        if t.dim() == 3:
+            sums = t.sum(dim=(1, 2), dtype=torch.int64).to(torch.float64)
+            np.save(d / f"{name}_plane_sums{suffix}.npy", sums.cpu().numpy())
 
 
 def crossing_edges(mask_u8, iso=127):
@@ -626,6 +650,9 @@ def run_gpu(args):
         timed[name] = {"ms_per_step": total_ms / args.steps, "stage_ms": stage_ms / args.steps,
                        "rounds": info["rounds"], "exchanges": info.get("exchanges", 0), "V": info["V"], "T": info["T"], "reached": gc, "tsum": gt, "vsum": gv,
                        "nseeds": len(seeds)}
+        if head and args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"threshold_mask": d_mask, "flood_mask": shard.interior(d_out),
+                                             "vertices": v, "triangles": f}, "" if world == 1 else f"_rank{rank}")
     head = timed["global"]
     ms_per_step = head["ms_per_step"]
     value = world * N / (ms_per_step * 1e-3) / 1e6
@@ -854,7 +881,13 @@ def main():
     ap.add_argument("--cpu-slices", type=int, default=0, help="reference arm: time a slab of this many slices instead "
                                                               "of the full volume (0 = full volume, the default)")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary 1024^3 / watershed measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the threshold mask, grown mask and mesh of the last "
+                                                          "timed step to DIR/*.npy (sampled, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,7 +1,8 @@
 """Pins the CPU oracle against every known-answer the reference holds for the hot path:
   - tests/test_bone_thresholding.py:51-185 and tests/test_segmentation_tools.py:137-160 (threshold)
   - samples/Cranium.inv3 mask_0/mask_1 (thresholds produced by the reference itself;
-    crop + whole-volume slice counts in tests/golden/cranium_crop.npz, generator
+    crop, whole masks and slice counts in tests/golden/cranium_crop.npz, a lattice and the
+    threshold-bound voxels of the whole matrix in tests/golden/cranium_sample.npz, generator
     tools/make_golden_cranium.py)
   - tests/test_segmentation_tools.py:17-51, :54-102 (flood fill), :105-134 (fill holes)
 MIP/MIDA/LMIP/contour-MIP have no reference test or golden: parity unpinned (checked
@@ -25,27 +26,38 @@ def test_threshold_cranium_crop(orc, cranium):
         assert 0 < int((got == 255).sum()) < got.size
 
 
-def test_threshold_cranium_full_if_reference_present(orc, cranium):
-    """Whole-volume check against the shipped masks; only where /root/reference exists."""
-    import sys
+def test_threshold_cranium_whole_volume_sample(orc, cranium):
+    """Whole-volume check against the shipped masks, on the stored sample of the matrix: a
+    lattice over every slice, and every voxel on (or one past) a bound of either threshold."""
     from pathlib import Path
-    src = Path("/root/reference/samples/Cranium.inv3")
-    if not src.exists():
-        pytest.skip("reference checkout not present (GPU box)")
-    sys.path.insert(0, str(Path(__file__).resolve().parents[1] / "tools"))
-    from make_golden_cranium import load_inv3
-    _, matrix, masks = load_inv3(src)
-    assert np.array_equal(matrix.astype(np.int64).sum(axis=(1, 2)), cranium["matrix_slice_sums"])
-    for i, (thr, m) in enumerate(masks):
-        got = np.zeros(matrix.shape, np.uint8)
-        orc.threshold(matrix, thr[0], thr[1], got, False)
-        assert np.array_equal(got, m[1:, 1:, 1:])
-        assert int((got == 255).sum()) == int(cranium[f"mask_{i}_count_full"])
-        assert np.array_equal((got == 255).sum(axis=(1, 2)), cranium[f"mask_{i}_slice_counts"])
+    smp = np.load(Path(__file__).resolve().parent / "golden" / "cranium_sample.npz")
+    shape = tuple(int(v) for v in cranium["full_shape"])
+    lat, step = smp["lattice"], tuple(int(s) for s in smp["lattice_step"])
+    on_lattice = tuple(slice(None, None, s) for s in step)
+    # the sample comes from the same matrix as the stored crop
+    crop = tuple(slice(int(a), int(b)) for a, b in cranium["crop"])
+    assert all(c.start % s == 0 for c, s in zip(crop, step))
+    in_crop = tuple(slice(c.start // s, -(-c.stop // s)) for c, s in zip(crop, step))
+    assert np.array_equal(lat[in_crop], cranium["matrix_crop"][on_lattice])
+    idx, val = smp["bound_index"], smp["bound_value"]
+    for i in (0, 1):
+        thr = cranium[f"thr_{i}"]
+        m = np.unpackbits(cranium[f"mask_{i}_bits_full"])[: int(np.prod(shape))].reshape(shape) * np.uint8(255)
+        assert int((m == 255).sum()) == int(cranium[f"mask_{i}_count_full"])
+        assert np.array_equal((m == 255).sum(axis=(1, 2)), cranium[f"mask_{i}_slice_counts"])
+        got = np.zeros(lat.shape, np.uint8)
+        orc.threshold(lat, thr[0], thr[1], got, False)
+        assert np.array_equal(got, m[on_lattice])
+        assert 0 < int((got == 255).sum()) < got.size
+        # the voxels on the bounds, as one row
+        got = np.zeros((1, 1, idx.size), np.uint8)
+        orc.threshold(val.reshape(got.shape), thr[0], thr[1], got, False)
+        assert np.array_equal(got.reshape(-1), m.reshape(-1)[idx])
+        assert (val == thr[0]).any() and (val == thr[0] - 1).any()
         # the reference's NumPy statements give the same thing
-        mm = np.zeros(m.shape, np.uint8)
-        orc.set_mask_threshold_numpy(matrix, mm, thr)
-        assert np.array_equal(mm[1:, 1:, 1:], got) and (mm[1:, 0, 0] == 1).all()
+        mm = np.zeros(tuple(s + 1 for s in lat.shape), np.uint8)
+        orc.set_mask_threshold_numpy(lat, mm, thr)
+        assert np.array_equal(mm[1:, 1:, 1:], m[on_lattice]) and (mm[1:, 0, 0] == 1).all()
 
 
 def test_threshold_reference_known_answers(orc):

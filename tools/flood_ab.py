@@ -1,5 +1,6 @@
 import sys, json, torch, numpy as np
-sys.path.insert(0,'/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from scipy.ndimage import generate_binary_structure
 from invesalius3_b200 import _lib, device as dev, phantom
 lib=_lib.load()

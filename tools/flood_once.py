@@ -1,5 +1,6 @@
 import sys, torch
-sys.path.insert(0, '/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from scipy.ndimage import generate_binary_structure
 from invesalius3_b200 import device as dev, phantom
 vol = phantom.ct((512, 512, 512), seed=2); seed = phantom.first_seed_in_range(vol, 256, 226, 3071)

@@ -1,7 +1,8 @@
 """One MIDA launch per configuration, for ncu captures: python tools/mida_once.py [n]"""
 import sys
+from pathlib import Path
 import torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from invesalius3_b200 import projection
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 1024
