@@ -255,6 +255,44 @@ int b2v_apply_view_matrix_transform(const void* volume, int dtype, int64_t dz, i
                                     int minterpol, double cval, void* out, int64_t odz, int64_t ody, int64_t odx,
                                     void* workspace, void* stream);
 
+/* ---- 3-D mask editor (invesalius/data/mask3d_editor_state.py) --------------------------------
+ * float64 in the reference's operation order throughout (no FMA, IEEE division and sqrt).
+ *
+ * b2v_mask_cut: invesalius_rs.mask_cut (mask_cut.rs:7-62). out: dense device uint8 [dz][dy][dx],
+ * edited in place. Each voxel > 127 at (z, y, x) maps p = (x sx, y sy, z sz, 1) through M and MV;
+ * when (M p)[3] > 0 and |MV p / (MV p)[3]| <= max_depth it becomes 0 if its screen position
+ * (px, py) = ((q0 / 2 + 0.5)(w - 1), (q1 / 2 + 0.5)(h - 1)) lies on the filter and
+ * filter[trunc py][trunc px] != 0, or if it lies off the filter and edit_mode == 0.
+ * filter: dense device uint8 [h][w] (may be NULL when h * w == 0). spacing_host = (sx, sy, sz),
+ * m_host / mv_host = 16 doubles row-major, all on the HOST. Does not synchronise. */
+int b2v_mask_cut(uint8_t* out, int64_t dz, int64_t dy, int64_t dx, const double* spacing_host, double max_depth,
+                 const uint8_t* filter, int64_t h, int64_t w, const double* m_host, const double* mv_host, int edit_mode,
+                 void* stream);
+/* The voxel box brush_mask.rs:24-31 visits for a sphere of `radius` at center_host = (cx, cy, cz)
+ * (millimetres) in a [dz][dy][dx] volume with spacing_host = (sx, sy, sz): box_host receives
+ * (z0, y0, x0, nz, ny, nx), all zero when the box is empty. Host only: no device work. */
+int b2v_brush_bbox(int64_t dz, int64_t dy, int64_t dx, const double* spacing_host, const double* center_host,
+                   double radius, int64_t* box_host);
+/* b2v_brush_mask: invesalius_rs.brush_mask_rs (brush_mask.rs:5-71) applied to the part of a
+ * [dz][dy][dx] volume held on the device as the box [oz, oz + bz) x [oy, oy + by) x [ox, ox + bx):
+ * out (and orig, when not NULL) are dense device uint8 [bz][by][bx] copies of that box. Voxels in
+ * both the box and b2v_brush_bbox's box with (dx^2 + dy^2) + dz^2 <= radius^2: edit_mode 1 sets
+ * those > 0 to 0; edit_mode 0 sets them to orig when orig > 0, or to 255 without orig; any other
+ * mode does nothing. Does not synchronise. */
+int b2v_brush_mask(uint8_t* out, const uint8_t* orig, int64_t bz, int64_t by, int64_t bx, int64_t oz, int64_t oy,
+                   int64_t ox, int64_t dz, int64_t dy, int64_t dx, const double* spacing_host, const double* center_host,
+                   double radius, int edit_mode, void* stream);
+/* b2v_polygons_raster: invesalius_rs.polygon2mask_rs (polygon_mask.rs:4-79) for k >= 1 polygons at
+ * once on a (w, h) screen. points: device float64 [total][2] (x, y); offsets: device int64 [k + 1],
+ * polygon p is points[offsets[p] .. offsets[p + 1]). Pixel (r < w, c < h) is the even-odd
+ * inside(px = r, py = c) OR-ed over the polygons (each inside its own bounding box), XOR negate.
+ * transpose == 0 writes out[r][c] (uint8 [w][h], polygon2mask_rs's layout); transpose != 0 writes
+ * out[c][r] (uint8 [h][w], the filter of b2v_mask_cut). workspace: b2v_polygons_workspace_bytes(k)
+ * device bytes. Does not synchronise. */
+int64_t b2v_polygons_workspace_bytes(int64_t k);
+int b2v_polygons_raster(const double* points, const int64_t* offsets, int64_t k, int64_t w, int64_t h, int transpose,
+                        int negate, uint8_t* out, void* workspace, void* stream);
+
 /* ---- marching cubes ---------------------------------------------------------------
  * Replaces the contour step of create_surface_piece, invesalius/data/surface_process.py:
  * 156-186 (vtkImageFlip about the origin + vtkContourFilter at iso 127 on the uint8 mask,

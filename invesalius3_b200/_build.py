@@ -78,11 +78,13 @@ def build_cuda(force: bool = False, verbose: bool = False) -> Path:
 
 
 def build_oracle(force: bool = False) -> Path:
-    """Compile the CPU oracle (test infrastructure only) via oracle/Makefile."""
-    r = subprocess.run(["make", "-C", str(ROOT / "oracle"), *(["-B"] if force else [])],
-                       capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"oracle build failed:\n{r.stdout}\n{r.stderr}")
+    """Compile the CPU oracle (test infrastructure only) via oracle/Makefile, and the 3-D mask
+    editor's restatement via oracle/mask_edit.mk."""
+    for recipe in ([], ["-f", "mask_edit.mk"]):
+        r = subprocess.run(["make", "-C", str(ROOT / "oracle"), *recipe, *(["-B"] if force else [])],
+                           capture_output=True, text=True)
+        if r.returncode != 0:
+            raise RuntimeError(f"oracle build failed:\n{r.stdout}\n{r.stderr}")
     return ROOT / "oracle" / "liboracle.so"
 
 

@@ -65,6 +65,11 @@ PROTOTYPES = {
     "b2v_count_regions": (cint, [vp, cint, i64, u32, vp, vp, vp]),
     "b2v_apply_view_matrix_transform": (cint, [vp, cint, i64, i64, i64, vp, vp, i64, cint, cint, dbl, vp, i64, i64, i64, vp,
                                                vp]),
+    "b2v_mask_cut": (cint, [vp, i64, i64, i64, vp, dbl, vp, i64, i64, vp, vp, cint, vp]),
+    "b2v_brush_bbox": (cint, [i64, i64, i64, vp, vp, dbl, vp]),
+    "b2v_brush_mask": (cint, [vp, vp, i64, i64, i64, i64, i64, i64, i64, i64, i64, vp, vp, dbl, cint, vp]),
+    "b2v_polygons_workspace_bytes": (i64, [i64]),
+    "b2v_polygons_raster": (cint, [vp, vp, i64, i64, i64, cint, cint, vp, vp, vp]),
     "b2v_mc_workspace_bytes": (i64, [i64, i64, i64]),
     "b2v_mc_count": (cint, [vp, cint, i64, i64, i64, dbl, vp, vp, C.POINTER(i64), C.POINTER(i64)]),
     "b2v_mc_emit": (cint, [vp, cint, i64, i64, i64, dbl, vp, f32, f32, f32, i32, i32, i32, cint, vp, vp, vp]),
